@@ -19,6 +19,9 @@ A step = ONE forward of the hot path (pack+conv1_1 -> conv trunk -> regression h
            with two separate models and with the launcher's shared trunk.
 Every rank also runs ONE fixed-seed image outside the timed region; rank 0 asserts that all ranks produced the same
 bytes (the rank != 0 weight path: reserve -> broadcast -> adopt).
+--dump-outputs DIR writes rank 0's ab maps of the last timed step to DIR/ab.npy (float32 [N,2,X,X]; only the leading
+images when the batch exceeds 60 MiB).  Weights and inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 The reference arm times the UNMODIFIED reference wrapper `ColorizeImageTorch.net_forward` (staged by
 `__graft_entry__.build()` into the git-ignored oracle/_ref/, kind "reference") on the host cores, looping single-image
 calls as the reference does (models/pytorch/model.py:139-141); without the staged copy it falls back to the CPU oracle
@@ -42,6 +45,7 @@ if ROOT not in sys.path:
 METRIC = "net_forward images/sec @256x256"   # --size 512 reports the same metric name with the size in config
 X = 256
 PER_GPU_BATCH = 64
+DUMP_BYTES = 60 << 20                        # --dump-outputs stays under 64 MB, .npy header included
 NCU_TRAFFIC_CSV = os.path.join(ROOT, "profiles", "r02_ncu_full_batch64_forward.csv")
 
 
@@ -475,6 +479,10 @@ def run_ours(args):
     clocks = sampler.finish(t_region0, t_region1) if sampler else None
     ms_step = ms_total / args.steps
     value = world * N / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        ab_last = out.cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "ab.npy"), ab_last[:DUMP_BYTES // ab_last[0].nbytes])
 
     # ---- per-op device times: separate untimed pass (events between the launches, PDL off by construction) ----
     ctx.set_profiling(True)
@@ -578,7 +586,12 @@ def main():
     ap.add_argument("--fast-fp16", action="store_true",
                     help="NOT the parity configuration: single-pass FP16 operands (1 MMA per product, ~6e-2 ab error)")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only: skip the e2e, config 4 and latency legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's ab maps to DIR/ab.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: use it with --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -1,11 +1,10 @@
 """CPU: the oracle against the committed golden vectors (generated from the UNMODIFIED
-reference by tests/golden/make_golden.py) and, when /root/reference is present, against
-the live reference module."""
+reference by the scripts in tests/golden/)."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import color_ref, lhn_ref, ref_shims, synth
+from oracle import color_ref, lhn_ref, synth
 from tests import util
 
 
@@ -80,20 +79,17 @@ def test_product_color_matches_oracle():
                           color_ref.lab2rgb_transpose(lab[..., :1].transpose(2, 0, 1), lab[..., 1:].transpose(2, 0, 1)))
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="/root/reference not present (GPU box)")
-def test_oracle_vs_live_reference(synth_sd):
-    model = ref_shims.import_reference_model()
-    net = model.SIGGRAPHGenerator(dist=True)
-    net.load_state_dict(synth_sd)
-    net.eval()
-    L, ab, m = util.small_batch(1, 64, seed=7)
-    reg, dist = net.forward(L[0], ab[0], m[0], 0.5)
-    (oreg, odist) = lhn_ref.lhn_forward(synth_sd, L, ab, m, 0.5, dist=True, ref_quirks=True)
-    assert util.maxabs(reg.detach(), oreg) < 1e-3                 # values are O(1e3) here (quirk q1)
-    assert util.maxabs(dist.detach(), lhn_ref.upsample4(odist)) < 1e-7
+def test_oracle_vs_reference_forward(synth_sd):
+    """The oracle against the reference's own SIGGRAPHGenerator(dist=True).forward, as recorded by
+    tests/golden/make_ref_forward_golden.py (same weights, one 64x64 synthetic image)."""
+    g = util.golden("ref_forward_64.npz")
+    (oreg, odist) = lhn_ref.lhn_forward(synth_sd, g["L"], g["ab"], g["mask"], 0.5, dist=True, ref_quirks=True)
+    assert util.maxabs(oreg, g["reg"]) < 1e-3                     # values are O(1e3) here (quirk q1)
+    y, x = g["dist_yx"]
+    assert util.maxabs(lhn_ref.upsample4(odist)[0][:, y, x], g["dist_at_yx"]) < 1e-7
     # state_dict key compatibility of the drop-in module
     from interactive_deep_colorization_b200.model import SIGGRAPHGeneratorB200
-    assert set(SIGGRAPHGeneratorB200(dist=True).state_dict().keys()) == set(net.state_dict().keys())
+    assert set(SIGGRAPHGeneratorB200(dist=True).state_dict().keys()) == set(g["state_dict_keys"].tolist())
 
 
 def test_global_stats_encode_pinned_to_reference_nnenc():
