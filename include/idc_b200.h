@@ -80,12 +80,8 @@ int idc_create(int device, int max_n, int h, int w, unsigned flags, idc_ctx** ou
  *   "split_k"       >= 1        K slices per tile on launches that cannot fill the machine
  *   "split_pairs"   0 / 1       run the split-K (small batch) launches as CTA pairs
  *   "split_bn128"   0 / 1       128-column tiles on the split-K path (default 1: half the reduction traffic per CTA)
- *   "halo_split"    0 / 1       halo-tile A operand on that path (experiment, measured slower; default 0)
- *   "chain"         0 / 1       the consecutive split-K layers as ONE launch with a grid barrier (measured equal; default 0)
- *   "prologue_sync2" 0 / 1      cluster barrier in front of the CTA pair's TMEM allocation (default 1; 0 is racecheck-dirty)
  *   "conv1_1_umma"  0 / 1       model1.0 on the tensor cores (default 1); 0 = the exact-FP32 CUDA-core kernel
- *   "direct_stores" 0 / 1       per-lane 16-byte stores instead of the warp-transposed ones
- *   "host_pipe"     0 / 1       idc_forward_host: chunked copy/compute overlap for batches >= 8
+ *   "host_pipe"     0 / 1      idc_forward_host: chunked copy/compute overlap for batches >= 8
  *   "pdl"           0 / 1       programmatic dependent launch between the kernels of one forward
  *   "side_dist"     0 / 1       batches <= 4: run the dist head (class + softmax) on a side stream / graph branch
  *   "tanh_scale"    110 / 100   regression head scale: tanh * 110 (model.py:175) or the Caffe nets' 100

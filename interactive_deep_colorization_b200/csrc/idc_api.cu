@@ -473,10 +473,6 @@ int plan_engines(Ctx* c) {
     CUDA_TRY(c, cudaMalloc(&c->splitk_ws, c->splitk_ws_floats * sizeof(float)));
     CUDA_TRY(c, cudaMalloc(&c->splitk_counters, sizeof(int) * 2 * (size_t)c->splitk_max_tiles));
     CUDA_TRY(c, cudaMemset(c->splitk_counters, 0, sizeof(int) * 2 * (size_t)c->splitk_max_tiles));
-    if (!c->chain_bar) {
-      CUDA_TRY(c, cudaMalloc(&c->chain_bar, 256));
-      CUDA_TRY(c, cudaMemset(c->chain_bar, 0, 256));
-    }
   }
   return IDC_OK;
 }
@@ -568,19 +564,8 @@ int run_forward(Ctx* c, int n, const float* L, const float* ab, const float* mas
   // 128-CTA launches of the main chain leave idle, instead of sitting between c8_3 and up9 on the critical path.
   const bool side_dist = c->opt.side_dist && !c->simt && out_dist && n <= 4 && !hp && !ev;
   bool forked = false;
-  // chained launches: not while per-op events are recorded, not on the chunked large-batch path
-  const bool use_chain = c->opt.chain && !c->simt && !ev && !hp && c->chain_bar;
   for (size_t oi = 0; oi < c->ops.size(); ++oi) {
     ConvOp& op = c->ops[oi];
-    if (use_chain && umma_op_chainable(c, op)) {
-      size_t oj = oi;
-      while (oj + 1 < c->ops.size() && oj + 1 - oi < 20 && umma_op_chainable(c, c->ops[oj + 1])) ++oj;
-      if (oj > oi) {
-        CUDA_TRY(c, umma_run_chain(c, (int)oi, (int)oj, n, st));
-        oi = oj;
-        continue;
-      }
-    }
     if (side_dist && op.kind == OP_CLASS && op.name == "class") {
       if (!c->s_side) {
         CUDA_TRY(c, cudaStreamCreateWithFlags(&c->s_side, cudaStreamNonBlocking));
@@ -709,9 +694,9 @@ int idc_set_option(idc_ctx* c, const char* name, int value) {
   if (!c || !name) return IDC_ERR_ARG;
   struct { const char* n; int* v; } tab[] = {
       {"halo", &c->opt.halo}, {"pairs", &c->opt.pairs}, {"mt", &c->opt.mt}, {"chunk_kb", &c->opt.chunk_kb},
-      {"split_k", &c->opt.split_k}, {"direct_stores", &c->opt.direct_stores}, {"host_pipe", &c->opt.host_pipe},
+      {"split_k", &c->opt.split_k}, {"host_pipe", &c->opt.host_pipe},
       {"pdl", &c->opt.pdl}, {"split_pairs", &c->opt.split_pairs}, {"tanh_scale", &c->opt.tanh_scale},
-      {"side_dist", &c->opt.side_dist}, {"split_bn128", &c->opt.split_bn128}, {"halo_split", &c->opt.halo_split}, {"prologue_sync2", &c->opt.prologue_sync2}, {"chain", &c->opt.chain}, {"conv1_1_umma", &c->opt.conv1_1_umma}};
+      {"side_dist", &c->opt.side_dist}, {"split_bn128", &c->opt.split_bn128}, {"conv1_1_umma", &c->opt.conv1_1_umma}};
   for (auto& t : tab)
     if (!strcmp(t.n, name)) {
       *t.v = value;
@@ -1452,7 +1437,6 @@ int idc_destroy(idc_ctx* c) {
   if (c->pts313) cudaFree(c->pts313);
   if (c->splitk_ws) cudaFree(c->splitk_ws);
   if (c->splitk_counters) cudaFree(c->splitk_counters);
-  if (c->chain_bar) cudaFree(c->chain_bar);
   if (c->w11_umma) cudaFree(c->w11_umma);
   if (c->d_reccs) cudaFree(c->d_reccs);
   if (c->gvec) cudaFree(c->gvec);

@@ -114,16 +114,11 @@ struct Options {
   int mt = -1;            // M-tiles per CTA tile on the <= 128-column layers (1 / 2)
   int chunk_kb = -1;      // k-blocks summed in TMEM before the FP32 round-to-nearest add
   int split_k = -1;       // K slices per tile on launches that cannot fill the machine
-  int direct_stores = 0;  // 1 = per-lane 16-byte stores instead of the warp-transposed ones
   int host_pipe = 1;      // idc_forward_host: chunked copy/compute overlap for batches >= 8
   int pdl = 1;            // programmatic dependent launch between the kernels of a forward
   int split_pairs = 1;    // cta_group::2 on the split-K (small batch) path
   int split_bn128 = 1;    // 128-column tiles on the split-K path (halves the partial-tile traffic of the reduction)
   int conv1_1_umma = 1;   // model1.0 on the tensor cores (one padded k-block); 0 = the FP32 CUDA-core kernel
-  int chain = 0;          // run consecutive same-shaped split-K layers as ONE launch with a grid barrier between layers
-  int prologue_sync2 = 1; // pairs: cluster barrier between barrier init and the cta_group::2 TMEM allocation (0: -3 us per click,
-                          // bit-identical results, but compute-sanitizer racecheck flags the allocation -> kept on)
-  int halo_split = 0;     // halo-tile A operand on the 128-column split-K path (stride-1 3x3 layers; experiment)
   int side_dist = 1;      // batch <= 4: run the dist head (class + softmax) on a side stream next to levels 9-10
   int tanh_scale = 110;   // regression head: tanh * 110 (model.py:175); the Caffe deploy nets use 100 (SURVEY q4)
 };
@@ -169,7 +164,6 @@ struct Ctx {
   // split-K workspace of the tcgen05 engine (sized by umma_plan_op, allocated after planning)
   float* splitk_ws = nullptr; size_t splitk_ws_floats = 0;
   int* splitk_counters = nullptr; int splitk_max_tiles = 0;
-  int* chain_bar = nullptr;      // grid-wide arrive counter of the chained launches (self-resetting)
   long long* dbgbuf = nullptr;   // experiments: per-CTA cycle counters of the last tcgen05 launch
   bool dbg_graph_timing = false; // experiments: events around the click graph launch (idc_debug_graph_timing)
   cudaEvent_t dbg_ev[2] = {nullptr, nullptr};
@@ -224,8 +218,6 @@ void umma_free_op(ConvOp& op);
 cudaError_t umma_run_op(Ctx* c, ConvOp& op, int n, float* out_ab_fused, float out_mult, cudaStream_t st, int img0 = 0,
                         int max_ctas = 0);   // max_ctas > 0: cap the persistent grid (side-branch launches)
 bool umma_op_uses_split_k(const ConvOp& op);
-bool umma_op_chainable(const Ctx* c, const ConvOp& op);   // may run inside a chained launch (see conv_body<..., CHAIN>)
-cudaError_t umma_run_chain(Ctx* c, int first, int last, int n, cudaStream_t st);   // ops[first..last] in ONE launch
 
 cudaError_t launch_conv1_1(Ctx* c, int n, const float* L, const float* ab, const float* mask,
                            float maskcent, cudaStream_t st, int img0 = 0);   // L/ab/mask: full arrays; images img0..img0+n

@@ -21,9 +21,8 @@
 //   store, or the fused model_out head).  Warp w owns TMEM lane quarter w%4 and column half (w-2)/4.
 //   Persistent grid = min(tiles, #SM).
 // * also in this file: CTA pairs (cta_group::2), the halo-tile A operand, deterministic split-K for launches that
-//   cannot fill the machine (128-column tiles; the CTA's own pieces never leave its registers), the chained launch
-//   (conv_body<..., CHAIN>: several layers, one launch, grid barrier) and conv1_1_umma_kernel (model1.0 as one padded
-//   k-block whose operand rows the threads write themselves).
+//   cannot fill the machine (128-column tiles; the CTA's own pieces never leave its registers) and
+//   conv1_1_umma_kernel (model1.0 as one padded k-block whose operand rows the threads write themselves).
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -63,7 +62,6 @@ struct UmmaParams {
   __half* out_hi;
   __half* out_lo;
   int Hout, Wout, Cout, os;
-  int store_mode;      // 0 = every lane stores its own row; 1 = warp-transposed through smem (default)
   float* out_f32;      // logits [M][out_ld] or null
   int out_ld;
   const float* wout;   // fused head weights [2][128] or null
@@ -75,7 +73,6 @@ struct UmmaParams {
   int n_amaps;         // entries of `amaps` (prefetched in the prologue)
   int max_ctas;        // host side only: grid cap for side-branch launches
   int halo_groups;     // HALO kernels: 64-channel input groups (K = 9 taps x halo_groups k-blocks); kblk = {-, B k-column, dy+1, dx+1}
-  int prologue_sync2;  // pairs: cluster barrier between barrier init and TMEM allocation (option, default 1)
   int img0;            // first image of this launch (n_img = img0 + images of the launch): idc_forward_host
                        // runs the last op in image chunks so that the D2H of a chunk overlaps the next one
 };
@@ -119,18 +116,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int* er
   while (!mbar_try_wait(bar, parity)) {
     if (clock64() - t0 > 6000000000LL) mbar_timeout(err, code);
   }
-}
-
-// Chain launches: poll side of the grid-wide arrive counter (bounded like every other wait).
-__device__ __forceinline__ void grid_wait(const int* bar, int target, int* err) {
-  int seen;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(bar) : "memory");
-  if (seen >= target) return;
-  const long long t0 = clock64();
-  do {
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(bar) : "memory");
-    if (seen < target && clock64() - t0 > 6000000000LL) mbar_timeout(err, 8);
-  } while (seen < target);
 }
 
 // one lane of a converged warp (warp-uniform control flow keeps descriptors / addresses in uniform
@@ -343,16 +328,11 @@ struct SmemPlan {
 // ------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------
-// CHAIN: one launch runs `nl` consecutive layers that share a tile configuration (the split-K layers of the interactive
-// path, conv3_1 ... conv8_3): barriers, TMEM and the operand ring stay alive, layer l+1's first weight tiles stream in
-// while layer l is still being reduced, and a grid-wide arrive / poll counter (`gridbar`) replaces the launch boundary:
-// a CTA's producer loads layer l+1's activations only after EVERY CTA has stored its part of layer l.
-template <int BN, int MT, int CG, bool SPLIT, bool HALO, bool CHAIN>
-__device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUtensorMap* blo_list,
-                                          const UmmaParams* plist, const int nl, int* gridbar) {
-  static_assert(!(HALO && CHAIN), "chained launches use per-tap boxes");
+// The body of umma_conv_kernel.  It stays a separate inlined function: written directly as the __global__ function's
+// body, ptxas allocates <128, 2, 2, false> with 24 B of stack and 48 B of spill stores instead of 16 B and 36 B.
+template <int BN, int MT, int CG, bool SPLIT, bool HALO>
+__device__ __forceinline__ void conv_body(const CUtensorMap& bmap_hi, const CUtensorMap& bmap_lo, const UmmaParams& p) {
   using SP = SmemPlan<BN, MT, CG, SPLIT, HALO>;
-  const UmmaParams& p0 = plist[0];
   constexpr int STAGES = SP::kStages;
   constexpr bool PAIR = CG == 2;
   extern __shared__ uint8_t smem_raw[];
@@ -376,19 +356,19 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
   float* s_red = reinterpret_cast<float*>(s_bar + 32);   // [128][2] fused-head partial sums, after the 256-byte barrier block
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long t_kernel0 = (IDC_CTA_COUNTERS && p0.dbgbuf) ? clock64() : 0;
+  const long long t_kernel0 = (IDC_CTA_COUNTERS && p.dbgbuf) ? clock64() : 0;
 
   // ---- one-time setup ----
-  if (!CHAIN && p0.wout) {
-    for (int i = threadIdx.x; i < 256; i += kThreads) s_head[i] = p0.wout[i];
-    if (threadIdx.x < 2) s_head[256 + threadIdx.x] = p0.bout[threadIdx.x];
+  if (p.wout) {
+    for (int i = threadIdx.x; i < 256; i += kThreads) s_head[i] = p.wout[i];
+    if (threadIdx.x < 2) s_head[256 + threadIdx.x] = p.bout[threadIdx.x];
   }
   const uint32_t cta_rank = PAIR ? cluster_ctarank() : 0u;
   const bool leader = cta_rank == 0;
   if (threadIdx.x == 32) {                          // descriptors are input-independent: fetch them during the prologue
-    prefetch_tmap(bhi_list);
-    if (SPLIT) prefetch_tmap(blo_list);
-    for (int i = 0; i < p0.n_amaps; ++i) prefetch_tmap(p0.amaps + i);
+    prefetch_tmap(&bmap_hi);
+    if (SPLIT) prefetch_tmap(&bmap_lo);
+    for (int i = 0; i < p.n_amaps; ++i) prefetch_tmap(p.amaps + i);
   }
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) {
@@ -407,9 +387,9 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   // Both CTAs of a pair are running before either executes the cta_group::2 TMEM allocation (it writes the base address
-  // into the peer's shared memory too).  Option prologue_sync2 = 0 drops this barrier: results stay bit-identical and a
-  // click gets 3 us shorter, but compute-sanitizer's racecheck then reports the allocation -- so it stays.
-  if (PAIR && p0.prologue_sync2) cluster_sync_all();
+  // into the peer's shared memory too).  Without this barrier results stay bit-identical and a click gets 3 us shorter,
+  // but compute-sanitizer's racecheck then reports the allocation -- so it stays.
+  if (PAIR) cluster_sync_all();
   if (warp == 1) {
     if (PAIR) {
       asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(s_tmem)),
@@ -431,7 +411,6 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
   if (warp != 0) pdl_wait();                         // warp 0 first requests its weight tiles (see the producer)
 
   long long t_wait_tfull_g = 0, t_drain_g = 0, t_epi_g = 0, t_splitk_g = 0, t_spin_g = 0;
-  const int n_layers = CHAIN ? nl : 1;
 
   if (warp < 4) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kCtrlRegs));
   if (warp == 0) {
@@ -440,21 +419,11 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
       int stage = 0;
       uint32_t phase = 0;
       uint32_t hcount = 0;                               // HALO: halo loads issued (slot = hcount & 1)
-      for (int l = 0; l < n_layers; ++l) {
-      const UmmaParams& p = plist[l];
-      const CUtensorMap& bmap_hi = bhi_list[l];
-      const CUtensorMap& bmap_lo = blo_list[l];
       const int tiles_per_img = p.tiles_y * p.tiles_x;
       const int S = p.split_k;
-      if (CHAIN && l + 1 < n_layers && elect_one()) {    // the next layer's descriptors: fetched a whole layer ahead
-        prefetch_tmap(bhi_list + l + 1);
-        if (SPLIT) prefetch_tmap(blo_list + l + 1);
-        for (int i = 0; i < plist[l + 1].n_amaps; ++i) prefetch_tmap(plist[l + 1].amaps + i);
-      }
       // Weights never depend on the previous layer: request the weight tiles of this CTA's first k-blocks BEFORE
-      // the dependency wait (pdl_wait / the chain's grid barrier), so they stream in while the predecessor drains.
-      // The stage's `full` barrier is armed with the byte count of the whole stage; the activation boxes follow
-      // after the wait.  (CHAIN: the ring position may still hold the previous layer's last k-blocks -> wait for it.)
+      // pdl_wait, so they stream in while the predecessor drains.  The stage's `full` barrier is armed with the byte
+      // count of the whole stage; the activation boxes follow after the wait.
       const int w0 = blockIdx.x / CG;
       int npre = 0;
       if (w0 < p.total_tiles * S) {
@@ -467,13 +436,10 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
         const int brow = cls * p.cout_pad + nt * BN + (int)cta_rank * (BN / CG);
         const int4* kb = p.kblk + cls * p.nkb;
         npre = kend - kbeg < STAGES ? kend - kbeg : STAGES;
-        int st = stage;
-        uint32_t ph = phase;
-        for (int i = 0; i < npre; ++i) {
-          if (CHAIN) mbar_wait(smem_u32(&empty_bar[st]), ph ^ 1, p.err, 1);
+        for (int i = 0; i < npre; ++i) {                  // the ring is still empty: k-block kbeg + i goes to stage i
           if (elect_one()) {
-            const uint32_t fb = smem_u32(&full_bar[st]);
-            const uint32_t sb = smem_u32(smem + st * SP::kStageBytes) + (SPLIT ? 2 : 1) * SP::kAStage;
+            const uint32_t fb = smem_u32(&full_bar[i]);
+            const uint32_t sb = smem_u32(smem + i * SP::kStageBytes) + (SPLIT ? 2 : 1) * SP::kAStage;
             const int kcol = HALO ? __ldg(kb + kbeg + i).y : (kbeg + i) * kBK;
             if (PAIR) {
               if (leader) mbar_expect_tx(fb, 2 * SP::kStageBytes); else mbar_arrive_rank0(fb);
@@ -486,15 +452,9 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
             }
           }
           __syncwarp();
-          if (++st == STAGES) { st = 0; ph ^= 1; }
         }
       }
-      if (!CHAIN || l == 0) {
-        pdl_wait();                                      // activations of the previous layer are complete and visible
-      } else if (w0 < p.total_tiles * S) {
-        grid_wait(gridbar, l * (int)gridDim.x, p.err);   // every CTA has stored its part of layer l-1 ...
-        asm volatile("fence.proxy.async;" ::: "memory");  // ... and TMA (async proxy) may read it
-      }
+      pdl_wait();                                       // activations of the previous layer are complete and visible
       for (int w = w0; w < p.total_tiles * S; w += gridDim.x / CG) {
         const int tile = w / S, ks = w - tile * S;
         const int kbeg = (ks * p.nkb) / S, kend = ((ks + 1) * p.nkb) / S;
@@ -590,7 +550,6 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
       }
-      }   // layers
     }
   } else if (warp == 1 && leader) {
     // =============================== MMA issuer (pairs: leader CTA only) ========
@@ -598,12 +557,10 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
       constexpr uint32_t idesc = make_idesc(BN, kBM * CG);
       int stage = 0;
       uint32_t phase = 0;
-      uint32_t cc = 0;                                   // chunk counter (persists across tiles and layers)
+      uint32_t cc = 0;                                   // chunk counter (persists across tiles)
       uint32_t hcount = 0;                               // HALO: halo tiles consumed
       long long t_wait_tempty = 0, t_wait_full = 0, t_first_full = 0;
       const long long t_start = clock64();
-      for (int l = 0; l < n_layers; ++l) {
-      const UmmaParams& p = plist[l];
       const int G = p.chunk_kb;
       const int S = p.split_k;
       for (int w = blockIdx.x / CG; w < p.total_tiles * S; w += gridDim.x / CG) {
@@ -691,9 +648,7 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
           }
         }
       }
-      }   // layers
-      if (IDC_CTA_COUNTERS && p0.dbgbuf && lane == 0) {
-        const UmmaParams& p = p0;
+      if (IDC_CTA_COUNTERS && p.dbgbuf && lane == 0) {
         p.dbgbuf[blockIdx.x * 16 + 0] = clock64() - t_start;
         p.dbgbuf[blockIdx.x * 16 + 1] = t_wait_tempty;
         p.dbgbuf[blockIdx.x * 16 + 2] = t_wait_full;
@@ -713,14 +668,10 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
     const int t_base = (MT == 2) ? half * BN : half * CH;   // its first TMEM column inside a chunk buffer
     uint32_t cc = 0;
     long long t_epi = 0, t_wait_tfull = 0, t_drain = 0, t_splitk = 0, t_spin = 0;
-    for (int l = 0; l < n_layers; ++l) {
-    const UmmaParams& p = plist[l];
     const int tiles_per_img = p.tiles_y * p.tiles_x;
     const int G = p.chunk_kb;
     const int S = p.split_k;
     int staged_key = -1;
-    if (CHAIN && blockIdx.x / CG >= p.total_tiles * S && l > 0 && et == 0)
-      grid_wait(gridbar, l * (int)gridDim.x, p.err);   // idle in this layer: still arrive only after the previous barrier
     for (int w = blockIdx.x / CG; w < p.total_tiles * S; w += gridDim.x / CG) {
       const int tile = w / S, ks = w - tile * S;
       const int kbeg = (ks * p.nkb) / S, kend = ((ks + 1) * p.nkb) / S;
@@ -941,29 +892,8 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
             for (int q = 0; q < 8; ++q) o[q] = make_float4(f[4 * q], f[4 * q + 1], f[4 * q + 2], f[4 * q + 3]);
           }
         }
-      } else if (p.store_mode == 0) {
-        // direct: every lane stores its own pixel row (one L1 transaction per lane per instruction)
-        const size_t opix =
-            ((size_t)(img * p.Hout + y * p.os + (cls >> 1)) * p.Wout + x * p.os + (cls & 1)) * p.Cout + n0 + c_base;
-#pragma unroll
-        for (int ch = 0; ch < CH; ch += 32) {
-          if (S > 1 && ((c_base + ch) >> 5) % S != ks) continue;
-          float f[32];
-          slab(ch, f);
-          uint32_t hw[16], lw[16];
-          split_pack<SPLIT>(f, hw, lw);
-          if (valid) {
-            uint4* oh = reinterpret_cast<uint4*>(p.out_hi + opix + ch);
-            uint4* ol = SPLIT ? reinterpret_cast<uint4*>(p.out_lo + opix + ch) : nullptr;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              oh[q] = make_uint4(hw[4 * q], hw[4 * q + 1], hw[4 * q + 2], hw[4 * q + 3]);
-              if (SPLIT) ol[q] = make_uint4(lw[4 * q], lw[4 * q + 1], lw[4 * q + 2], lw[4 * q + 3]);
-            }
-          }
-        }
       } else {
-        // warp-transposed (default): the warp's 32 rows x 64 bytes go through a private 2 KB smem tile
+        // activation store, warp-transposed: the warp's 32 rows x 64 bytes go through a private 2 KB smem tile
         // (XOR-swizzled, conflict-free both ways) so that each store instruction writes 8 pixel rows x 64
         // contiguous bytes instead of 32 rows x 16 bytes -- 4x fewer L1 transactions.  Store instruction i of a
         // slab covers rows i*8 + lane/4 of this warp's 32 rows; rows outside the image get a null pointer.
@@ -1023,25 +953,11 @@ __device__ __forceinline__ void conv_body(const CUtensorMap* bhi_list, const CUt
         }
       }
     }
-    if (CHAIN) {
-      // grid barrier, arrive side: this CTA's part of layer l is stored (and its split-K counters are released)
-      asm volatile("bar.sync 1, 256;" ::: "memory");
-      if (et == 0) {
-        __threadfence();
-        const int old = atomicAdd(gridbar, 1);
-        if (l == n_layers - 1 && old == n_layers * (int)gridDim.x - 1) {   // last arrival of the launch: reset for the next one
-          *gridbar = 0;
-          __threadfence();
-        }
-      }
-    }
-    }   // layers
     t_wait_tfull_g = t_wait_tfull; t_drain_g = t_drain; t_epi_g = t_epi; t_splitk_g = t_splitk; t_spin_g = t_spin;
   }
 
   // ---- teardown ----
-  if (IDC_CTA_COUNTERS && p0.dbgbuf && warp == 4 && lane == 0) {
-    const UmmaParams& p = p0;
+  if (IDC_CTA_COUNTERS && p.dbgbuf && warp == 4 && lane == 0) {
     p.dbgbuf[blockIdx.x * 16 + 3] = t_wait_tfull_g;
     p.dbgbuf[blockIdx.x * 16 + 4] = t_drain_g;
     p.dbgbuf[blockIdx.x * 16 + 5] = t_epi_g;
@@ -1066,20 +982,7 @@ template <int BN, int MT, int CG, bool SPLIT, bool HALO = false>
 __global__ void __launch_bounds__(kThreads, 1)
 umma_conv_kernel(const __grid_constant__ CUtensorMap bmap_hi, const __grid_constant__ CUtensorMap bmap_lo,
                  const __grid_constant__ UmmaParams p) {
-  conv_body<BN, MT, CG, SPLIT, HALO, false>(&bmap_hi, &bmap_lo, &p, 1, nullptr);
-}
-
-// a run of consecutive layers in one launch (see conv_body); everything lives in the constant bank
-constexpr int kChainMax = 20;
-struct ChainParams {
-  CUtensorMap bhi[kChainMax], blo[kChainMax];
-  UmmaParams layer[kChainMax];
-  int nl;
-  int* gridbar;
-};
-template <int BN, int MT, int CG, bool SPLIT>
-__global__ void __launch_bounds__(kThreads, 1) umma_chain_kernel(const __grid_constant__ ChainParams P) {
-  conv_body<BN, MT, CG, SPLIT, false, true>(P.bhi, P.blo, P.layer, P.nl, P.gridbar);
+  conv_body<BN, MT, CG, SPLIT, HALO>(bmap_hi, bmap_lo, p);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1422,7 +1325,6 @@ int umma_plan_op(Ctx* c, ConvOp& op) {
     const int t = ceil_div(op.Wl, wb) * ceil_div(op.Hl, hb);
     if (t < best) { best = t; op.wbox = wb; op.hbox = hb; }
   }
-  bool halo_shape = false;
   // HALO: stride-1 3x3 convs of one source with 128 output columns per tile (c2_2, c9_2, c10_2: the layers that are
   // shared-memory-bandwidth bound with per-tap boxes) load one 18x10-pixel halo tile per 64 input channels instead of
   // one box per tap, when the launch fills the machine.  Measured at 64 x 256^2: c2_2 0.76 -> 0.63 ms, c9_2 0.76 ->
@@ -1439,7 +1341,6 @@ int umma_plan_op(Ctx* c, ConvOp& op) {
       else seen |= 1u << ((tp.ty + 1) * 3 + tp.tx + 1);
     }
     if (ok && (seen != 0x1FFu || op.src[op.taps[0][0].src].cin % kBK)) ok = false;
-    halo_shape = ok;                     // a stride-1 3x3 conv of one source: the split-K path may still pick halo tiles
     if (ok && !(op.bn_tile == 128 || (mode >= 3 && op.bn_tile == 64))) ok = false;
     if (ok) {   // only launches that fill the machine (the split-K path decides for itself below)
       const long T = (long)c->max_n * ceil_div(op.Hl, 16) * ceil_div(op.Wl, 8) * (op.cout_pad / op.bn_tile);
@@ -1509,14 +1410,6 @@ int umma_plan_op(Ctx* c, ConvOp& op) {
         if (S3 > 4) S3 = 4;                                // 128 columns = 4 pieces of 32
         if (c->opt.split_k >= 1 && c->opt.split_k <= S3) S3 = c->opt.split_k;
         if (S3 >= 2) { op.bn_tile = 128; S = S3; Tw = T3 * 2; }
-        // ... and with 128 columns the stride-1 3x3 layers can take the halo-tile A operand: a K slice of whole input
-        // groups (9 taps each) loads ONE 18x10-pixel halo per group instead of 9 boxes of 128 pixels, which cuts the
-        // L2 -> SM operand traffic of a slice from 48 to ~21 KB per k-block (option halo_split).
-        if (S3 >= 2 && c->opt.halo_split && halo_shape && nkb % 9 == 0 && (nkb / 9) % S3 == 0 &&
-            ceil_div(op.Hl, 16) * ceil_div(op.Wl, 8) == ty * tx) {
-          pl->halo = true;
-          op.wbox = 8; op.hbox = 16;
-        }
       }
     }
     pl->split_k = S;
@@ -1642,10 +1535,7 @@ int umma_plan_op(Ctx* c, ConvOp& op) {
     q.Hout = ob.H; q.Wout = ob.W; q.Cout = ob.C; q.os = op.os;
   }
   if (op.fuse_out_head) { q.wout = c->wout; q.bout = c->bout; }
-  q.store_mode = 1;
-  if (c->opt.direct_stores) q.store_mode = 0;
   q.err = c->d_err;
-  q.prologue_sync2 = c->opt.prologue_sync2;
   q.img0 = 0;
   q.dbgbuf = nullptr;
   return IDC_OK;
@@ -1665,12 +1555,11 @@ bool umma_op_uses_split_k(const ConvOp& op) {
   return pl && pl->split_k > 1;
 }
 
-// launch parameters of one op for `n` images (shared by the single-op and the chained launch)
-static cudaError_t umma_prepare(Ctx* c, ConvOp& op, int n, float* out_ab_fused, float out_mult, int img0, int max_ctas,
-                                UmmaParams& prm) {
+cudaError_t umma_run_op(Ctx* c, ConvOp& op, int n, float* out_ab_fused, float out_mult, cudaStream_t st, int img0,
+                        int max_ctas) {
   UmmaPlan* pl = static_cast<UmmaPlan*>(op.umma_plan);
   if (!pl) return cudaErrorInvalidValue;
-  prm = pl->prm;
+  UmmaParams prm = pl->prm;
   prm.max_ctas = (max_ctas > 0 && pl->split_k == 1) ? (max_ctas / pl->cg) * pl->cg : 0;   // split-K needs all items co-resident
   prm.img0 = img0;
   prm.n_img = img0 + n;
@@ -1686,72 +1575,6 @@ static cudaError_t umma_prepare(Ctx* c, ConvOp& op, int n, float* out_ab_fused, 
   if (pl->split_k > 1 && (!prm.ws || !prm.counters)) return cudaErrorInvalidValue;
   prm.out_mult = out_mult;
   if (op.fuse_out_head && !out_ab_fused) return cudaErrorInvalidValue;
-  return cudaSuccess;
-}
-
-// Chain launches (conv_body<..., CHAIN>): consecutive ops that all run as 128-column split-K CTA pairs with per-tap
-// boxes and write an ordinary activation -- at 256^2 / batch 1 that is conv3_1 ... conv8_3, 18 of the 26 conv launches.
-bool umma_op_chainable(const Ctx* c, const ConvOp& op) {
-  const UmmaPlan* pl = static_cast<const UmmaPlan*>(op.umma_plan);
-  return pl && !c->fast && op.bn_tile == 128 && pl->mt == 1 && pl->cg == 2 && pl->split_k > 1 && !pl->halo &&
-         !op.fuse_out_head && !op.out_f32 && op.out_buf >= 0;
-}
-
-cudaError_t umma_run_chain(Ctx* c, int first, int last, int n, cudaStream_t st) {
-  const int nl = last - first + 1;
-  if (nl < 2 || nl > kChainMax || !c->chain_bar) return cudaErrorInvalidValue;
-  ChainParams P;                                         // 10 KB of kernel parameters, copied by the launch itself
-  int grid = 0, dev = 0;
-  for (int k = 0; k < nl; ++k) {
-    ConvOp& op = c->ops[first + k];
-    if (!umma_op_chainable(c, op)) return cudaErrorInvalidValue;
-    UmmaPlan* pl = static_cast<UmmaPlan*>(op.umma_plan);
-    cudaError_t e = umma_prepare(c, op, n, nullptr, (float)c->opt.tanh_scale, 0, 0, P.layer[k]);
-    if (e != cudaSuccess) return e;
-    P.layer[k].dbgbuf = nullptr;
-    P.bhi[k] = pl->bmap_hi; P.blo[k] = pl->bmap_lo;
-    const long items = (long)P.layer[k].total_tiles * P.layer[k].split_k;
-    if (items * 2 > pl->num_sms) return cudaErrorInvalidValue;       // every work item of every layer must be resident
-    if (items * 2 > grid) grid = (int)items * 2;
-    dev = pl->dev;
-  }
-  P.nl = nl;
-  P.gridbar = c->chain_bar;
-  using SP = SmemPlan<128, 1, 2, true, false>;
-  static unsigned long long attr_devs = 0;
-  if (dev >= 64 || !(attr_devs & (1ull << dev))) {
-    cudaError_t e = cudaFuncSetAttribute(umma_chain_kernel<128, 1, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SP::kTotal);
-    if (e != cudaSuccess) return e;
-    if (dev < 64) attr_devs |= 1ull << dev;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = SP::kTotal;
-  cfg.stream = st;
-  cudaLaunchAttribute at[2];
-  int na = 0;
-  at[na].id = cudaLaunchAttributeClusterDimension;
-  at[na].val.clusterDim.x = 2; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
-  ++na;
-  if (pdl_take(c)) {
-    at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.attrs = at;
-  cfg.numAttrs = na;
-  c->launch_count++;
-  return cudaLaunchKernelEx(&cfg, umma_chain_kernel<128, 1, 2, true>, P);
-}
-
-cudaError_t umma_run_op(Ctx* c, ConvOp& op, int n, float* out_ab_fused, float out_mult, cudaStream_t st, int img0,
-                        int max_ctas) {
-  UmmaPlan* pl = static_cast<UmmaPlan*>(op.umma_plan);
-  if (!pl) return cudaErrorInvalidValue;
-  UmmaParams prm;
-  cudaError_t pe = umma_prepare(c, op, n, out_ab_fused, out_mult, img0, max_ctas, prm);
-  if (pe != cudaSuccess) return pe;
   c->launch_count++;
   const bool split = !c->fast;
   const bool pdl = pdl_take(c);

@@ -20,8 +20,8 @@ class LhnContext(object):
 
     def __init__(self, device=0, max_n=1, H=256, W=256, dist=False, engine="tcgen05", fast_fp16=False,
                  global_hints=False, use_graph=True, keep_conv10=False, caffe313=False, options=None):
-        """options: {name: int} plan-time switches, see include/idc_b200.h: idc_set_option
-        (halo, pairs, mt, chunk_kb, split_k, split_pairs, direct_stores, host_pipe, pdl)."""
+        """options: {name: int} plan-time switches; the names and values are listed at idc_set_option in
+        include/idc_b200.h."""
         self.lib = _lib.load()
         flags = 0
         if dist:

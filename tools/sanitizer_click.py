@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """GPU tool for compute-sanitizer: a few clicks through the whole interactive path (resident image, announced click,
-tensor-core conv1_1, 128-column split-K pairs, chained launch on the second context) at 64x64 -- small enough for
-memcheck / racecheck to finish in minutes.
+tensor-core conv1_1, 128-column split-K pairs) at 64x64 -- small enough for memcheck / racecheck to finish in
+minutes.  Plan options given as opt:val pairs apply to the context.
 
     compute-sanitizer --tool memcheck python tools/sanitizer_click.py [size] [opt:val,...]
 """
@@ -21,27 +21,21 @@ EXTRA = {kv.split(":")[0]: int(kv.split(":")[1]) for kv in (sys.argv[2].split(",
 sd = synth.torch_state_dict(1234)
 L, ab, m = synth.synthetic_batch(1, X, seed=0, max_hints=0)
 ab, m = ab.copy(), m.copy()
-outs = []
-for opts in ({}, {"chain": 1}):
-    opts = dict(opts, **EXTRA)
-    ctx = util.make_ctx(sd, X, X, max_n=1, dist=True, options=opts)
-    ctx.set_dist_resident(True)
-    buf = ctx.click_buffers(1)
-    buf["L_mc"][...] = L
-    ctx.set_image(buf["L_mc"])
-    rs = np.random.RandomState(0)
-    a1, m1 = ab.copy(), m.copy()
-    for i in range(3):
-        loc = rs.randint(8, X - 8, 2)
-        CI.put_point(a1[0], m1[0], loc, 2, rs.uniform(-80, 80, 2))
-        buf["ab"][...] = a1; buf["mask"][...] = m1
-        y4, x4 = int(loc[0]) // 4, int(loc[1]) // 4
-        ctx.set_click(0, y4, x4, 5)
-        r = ctx.forward_host(None, buf["ab"], buf["mask"], 0.5, want_rgb=True, want_abq=True, out_ab=buf["out_ab"],
-                             out_rgb=buf["out_rgb"], out_abq=buf["out_abq"])
-        pmf = ctx.fetch_dist(0, y4, x4)
-        cen, conf, it = ctx.ab_reccs(0, y4, x4, K=5)
-    outs.append((r["ab"].copy(), pmf.copy(), cen.copy()))
-    ctx.close()
-assert np.array_equal(outs[0][0], outs[1][0]) and np.array_equal(outs[0][1], outs[1][1]) and np.array_equal(outs[0][2], outs[1][2])
-print("sanitizer_click: %dx%d, 2 contexts x 3 clicks done; chain == per-layer launches: True; pmf sum %.6f" % (X, X, float(outs[0][1].sum())))
+ctx = util.make_ctx(sd, X, X, max_n=1, dist=True, options=EXTRA)
+ctx.set_dist_resident(True)
+buf = ctx.click_buffers(1)
+buf["L_mc"][...] = L
+ctx.set_image(buf["L_mc"])
+rs = np.random.RandomState(0)
+for i in range(3):
+    loc = rs.randint(8, X - 8, 2)
+    CI.put_point(ab[0], m[0], loc, 2, rs.uniform(-80, 80, 2))
+    buf["ab"][...] = ab; buf["mask"][...] = m
+    y4, x4 = int(loc[0]) // 4, int(loc[1]) // 4
+    ctx.set_click(0, y4, x4, 5)
+    ctx.forward_host(None, buf["ab"], buf["mask"], 0.5, want_rgb=True, want_abq=True, out_ab=buf["out_ab"],
+                     out_rgb=buf["out_rgb"], out_abq=buf["out_abq"])
+    pmf = ctx.fetch_dist(0, y4, x4)
+    ctx.ab_reccs(0, y4, x4, K=5)
+ctx.close()
+print("sanitizer_click: %dx%d, 3 clicks done; pmf sum %.6f" % (X, X, float(pmf.sum())))
